@@ -23,7 +23,9 @@ headline.
 
 Launch: python bench.py [--gpus N --steps K --warmup W] (N > 1 under torch.distributed.run, one rank per
 GPU).  `--impl reference` times the CPU port of the reference's own self-play worker (oracle/) on the host
-cores instead.  Prints ONE JSON line on rank 0.
+cores instead.  Prints ONE JSON line on rank 0.  `--dump-outputs DIR` also writes what the last timed step computed
+(the games it finished) as .npy files; the inputs (weights, engine seed, warm-start profile) are fixed, so two builds
+can be compared output for output.
 """
 import argparse
 import json
@@ -178,6 +180,50 @@ def run_reference(args):
     _emit(json.dumps(line))
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, games, step_stats):
+    """--dump-outputs: the games the timed engine finished in its last step, as Engine.poll() hands them to a caller, sorted
+    by game id, one array per field: `game_*` per game, `ply_*` per ply (`ply_game` indexes the game arrays), bitboards as
+    0/1 planes over the 64 squares; `step_counts` = games finished, expansions, simulations, plies and waves of that step.
+    Ids and counters are float64, planes, visit counts and search values float32.  Should the arrays exceed DUMP_MAX_BYTES,
+    a seeded sample of whole games is written instead."""
+    import numpy as np
+
+    def planes(*boards):
+        b = np.array(boards, dtype=np.uint64).T.reshape(-1, len(boards), 1)
+        return ((b >> np.arange(64, dtype=np.uint64)) & np.uint64(1)).astype(np.float32)
+
+    def nbytes(g):
+        return 8 * 10 + 4 * 128 + len(g["plies"]) * (8 + 4 * (128 + 64 + 7))
+
+    games = sorted(games, key=lambda g: g["game_id"])
+    if sum(nbytes(g) for g in games) > DUMP_MAX_BYTES:
+        keep, total = [], 0
+        for i in np.random.default_rng(0).permutation(len(games)):
+            if total + nbytes(games[i]) <= DUMP_MAX_BYTES:
+                keep.append(i)
+                total += nbytes(games[i])
+        games = [games[i] for i in sorted(keep)]
+    out = {"game_id": np.array([g["game_id"] for g in games], dtype=np.float64)}
+    for k in ("winner", "black_z", "expansions", "simulations", "resign_enabled", "resigned_mask", "turn", "table_nodes"):
+        out["game_" + k] = np.array([g[k] for g in games], dtype=np.float64)
+    out["game_n_plies"] = np.array([len(g["plies"]) for g in games], dtype=np.float64)
+    out["game_final_board"] = planes([g["black"] for g in games], [g["white"] for g in games]).reshape(len(games), 2, 64)
+    plies = [p for g in games for p in g["plies"]]
+    out["ply_game"] = np.repeat(np.arange(len(games), dtype=np.float64), out["game_n_plies"].astype(np.int64))
+    out["ply_board"] = planes([p["own"] for p in plies], [p["enemy"] for p in plies]).reshape(len(plies), 2, 64)
+    out["ply_visits"] = np.array([p["N"] for p in plies], dtype=np.float32).reshape(len(plies), 64)
+    for k in ("action", "pid", "loops", "recorded", "waves", "n", "q"):
+        out["ply_" + k] = np.array([p[k] for p in plies], dtype=np.float32)
+    out["step_counts"] = np.array([step_stats[k] for k in ("games_finished", "expansions", "simulations", "plies", "waves")],
+                                  dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_config(args):
     """the workload both arms are measured on (identical in the `--impl reference` line)"""
     c = dict(workload="selfplay ch5 net (256x10, random-init) G=%d games/GPU sims=%d K=8 c_puct=5 vl=3 noise=0.25 tau_turn=4 "
@@ -205,7 +251,11 @@ def main():
     ap.add_argument("--groups", type=int, default=0, help="engine overlap groups (0 = auto, 1 = no overlap: clean per-kernel timing)")
     ap.add_argument("--full-games", type=int, default=0, metavar="G",
                     help="calibration: play G complete games from a cold start and write gpurun_out/full_games.json")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the games the timed engine finished in its last step as DIR/<name>.npy (b200 arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     PLAY_KW["simulation_num_per_move"] = args.sims
     if args.solver:  # ch5.yml's default solver settings instead of the benchmark configuration (solver off)
         PLAY_KW["use_solver_turn"] = PLAY_KW["use_solver_turn_in_simulation"] = 50
@@ -299,7 +349,14 @@ def main():
         dist.barrier()
     torch.cuda.synchronize()
     sampler.start()
-    eng.run(max_waves=args.steps * wps)
+    # the last step runs on its own, after the games finished so far are taken off the engine's queue, so that what
+    # Engine.poll() returns afterwards is exactly what the last step computed (--dump-outputs)
+    if args.steps > 1:
+        eng.run(max_waves=(args.steps - 1) * wps)
+    while eng.poll_raw()[1]:
+        pass
+    s_last = eng.stats()
+    eng.run(max_waves=wps)
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
@@ -307,8 +364,10 @@ def main():
     s1 = eng.stats()
     d = {k: s1[k] - s0[k] for k in s1}
     run_ms = d["run_ms"]
-    eng.poll()
+    last_games = eng.poll()
     eng.close()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_games, {k: s1[k] - s_last[k] for k in s1})
     # roofline leg: the same workload with ONE slot group, so that the CUDA events around each tower launch bracket
     # exactly that kernel (with two groups a launch's events also contain the wait for the other group's launch)
     eng1 = make_engine(1, 20260922)

@@ -44,6 +44,38 @@ def test_reference_arm_line_and_shared_config():
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and "windows" in cb["sample"]
 
 
+def test_dump_outputs_writes_float_arrays_of_the_polled_games(tmp_path, monkeypatch):
+    """--dump-outputs: Engine.poll()'s games as float32 / float64 arrays sorted by game id, bitboards as exact 0/1 planes,
+    and a seeded sample of whole games when the set exceeds the size cap"""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+
+    def game(gid, n_plies):
+        ply = dict(own=0x0000000810000000, enemy=0x8000001008000001, N=np.arange(64), action=19, pid=1, loops=1, recorded=True,
+                   n=10.0, q=0.25, waves=50)
+        return dict(game_id=gid, black=0xFFFF000000000000, white=0xFFFF, winner=2, black_z=-1, expansions=300, simulations=400,
+                    resign_enabled=False, resigned_mask=0, turn=60, black_net=0, table_nodes=77, plies=[dict(ply) for _ in range(n_plies)])
+    games = [game(7, 3), game(2, 5), game(11, 1)]
+    stats = dict(games_finished=3, expansions=900, simulations=1200, plies=9, waves=50, run_ms=12.5)
+    bench.dump_outputs(str(tmp_path / "all"), games, stats)
+    load = lambda d, name: np.load(str(tmp_path / d / (name + ".npy")))   # noqa: E731
+    assert all(load("all", f[:-4]).dtype in (np.float32, np.float64) for f in os.listdir(tmp_path / "all"))
+    assert load("all", "game_id").tolist() == [2, 7, 11] and load("all", "game_n_plies").tolist() == [5, 3, 1]
+    assert load("all", "ply_game").tolist() == [0] * 5 + [1] * 3 + [2]
+    board = load("all", "ply_board")
+    assert board.shape == (9, 2, 64) and np.flatnonzero(board[0, 1]).tolist() == [0, 27, 36, 63]
+    assert np.flatnonzero(load("all", "game_final_board")[0, 0]).tolist() == list(range(48, 64))
+    assert np.array_equal(load("all", "ply_visits")[4], np.arange(64)) and load("all", "ply_q")[0] == np.float32(0.25)
+    assert load("all", "step_counts").tolist() == [3, 900, 1200, 9, 50]
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 8000)
+    bench.dump_outputs(str(tmp_path / "cut"), games, stats)
+    kept = load("cut", "game_id").tolist()
+    assert 1 <= len(kept) < 3 and kept == sorted(kept) and len(load("cut", "ply_game")) == sum(load("cut", "game_n_plies"))
+    bench.dump_outputs(str(tmp_path / "cut2"), games, stats)
+    assert load("cut2", "game_id").tolist() == kept
+
+
 def test_reference_arm_under_torchrun_prints_one_line_from_rank_0():
     """the driver launches the reference arm like the B200 arm (torchrun, one rank per GPU): rank 0 alone measures and prints,
     the other ranks exit 0 without work"""

@@ -2,6 +2,7 @@
 .force-sim override (worker/self_play.py:262-272), resignation-threshold auto-tuner (:219-260), GGF move text
 (:275-299, lib/ggf.py), config overlay of the reference's YAML structure, evaluation play-config defaults
 (config.py:103-113), rank-strided game ids."""
+import json
 import os
 import types
 
@@ -176,157 +177,115 @@ def test_match_verdict_follows_the_sequential_reference():
     assert match_verdict([0] * 5 + [1] * 5, 10, 0.55) == (False, 0.0, 5)
 
 
-def test_ggf_text_matches_reference_module(tmp_path):
-    """lib/ggf.py of the reference (importable as it is: stdlib only) against the mirror: square names both ways, the
-    record line for a fixed date, and MoveHistory's pass insertion (worker/self_play.py:275-299) against the worker's
-    _ggf_of.  Runs where the reference checkout exists."""
-    import oracle.ref_shims.install as shims
-    if not shims.available():
-        pytest.skip("reference sources not present")
-    shims.install()
+@pytest.fixture(scope="module")
+def ref_host(golden_dir):
+    """what the unmodified reference returned for the cases below (tests/golden/make_golden_standalone.py)"""
+    with open(os.path.join(golden_dir, "ref_host.json")) as f:
+        return json.load(f)
+
+
+def test_ggf_text_matches_reference_module(tmp_path, ref_host):
+    """lib/ggf.py of the reference against the mirror: square names both ways, the record line for a fixed date, and
+    MoveHistory's pass insertion (worker/self_play.py:275-299) against the worker's _ggf_of."""
     from datetime import datetime
-    from reversi_zero.lib import ggf as ref
     from reversi_zero_b200.lib import ggf as mine
-    for a in list(range(64)) + [None]:
-        mv = ref.convert_action_to_move(a)
-        assert mine.convert_action_to_move(a) == mv and mine.convert_move_to_action(mv) == ref.convert_move_to_action(mv) == a
-    assert mine.convert_move_to_action("f5") == ref.convert_move_to_action("f5") == 44      # test/lib/test_ggf.py:32-43
-    dt = datetime(2026, 9, 22, 13, 5, 9)
-    moves = ["C4/2.5/10.0", "C3/-5.0/7.0", "PA", "C2/0.0/3.0"]
-    for kw in (dict(), dict(result="+12.0", think_time_sec=125)):
-        assert mine.make_ggf_string("RAZ", "RAZ", dt=dt, moves=moves, **kw) == ref.make_ggf_string("RAZ", "RAZ", dt=dt, moves=moves, **kw)
-    assert mine.make_ggf_string(dt=dt) == ref.make_ggf_string(dt=dt)
+    ref = ref_host["ggf"]
+    assert ref["actions"] == list(range(64)) + [None]
+    for a, mv, back in zip(ref["actions"], ref["moves"], ref["move_to_action"]):
+        assert mine.convert_action_to_move(a) == mv and mine.convert_move_to_action(mv) == back == a
+    assert mine.convert_move_to_action("f5") == ref["f5"] == 44      # test/lib/test_ggf.py:32-43
+    dt = datetime(*ref["dt"])
+    for kw, want in zip((dict(), dict(result="+12.0", think_time_sec=125)), ref["with_moves"], strict=True):
+        assert mine.make_ggf_string("RAZ", "RAZ", dt=dt, moves=ref["record_moves"], **kw) == want
+    assert mine.make_ggf_string(dt=dt) == ref["dt_only"]
     # without dt both stamp "now" (UTC, naive): same layout, the "%Z" part empty
-    assert mine.make_ggf_string()[: len("(;GM[Othello]PC[RAZSelf]DT[")] == ref.make_ggf_string()[: len("(;GM[Othello]PC[RAZSelf]DT[")]
-    assert mine.make_ggf_string().split("DT[")[1].split("]")[0].endswith(".") and ref.make_ggf_string().split("DT[")[1].split("]")[0].endswith(".")
+    assert mine.make_ggf_string()[: len("(;GM[Othello]PC[RAZSelf]DT[")] == ref["now"][: len("(;GM[Othello]PC[RAZSelf]DT[")]
+    assert mine.make_ggf_string().split("DT[")[1].split("]")[0].endswith(".") and ref["now"].split("DT[")[1].split("]")[0].endswith(".")
     # MoveHistory: black C4, white C3, white again (black had to pass), black resigns
-    from reversi_zero.worker.self_play import MoveHistory
-    from reversi_zero.agent.player import ActionWithEvaluation
-    from reversi_zero.env.reversi_env import Player
-    mh = MoveHistory()
     P = _cabi.Ply
     plies = []
     for action, player, q, n in ((19, 1, 0.25, 10.0), (18, 2, -0.5, 7.0), (17, 2, 0.0, 3.0), (-1, 1, 0.0, 0.0)):
-        env = types.SimpleNamespace(next_player=Player.black if player == 1 else Player.white)
-        mh.move(env, ActionWithEvaluation(None if action < 0 else action, n, q))
         p = P(); p.action, p.player, p.q, p.n = action, player, q, n
         plies.append(p)
     cfg, w = make_worker(tmp_path)
-    theirs, ours = mh.make_ggf_string("RAZ", "RAZ"), w._ggf_of(None, plies)
-    assert theirs.split("BO[")[1] == ours.split("BO[")[1]            # everything after the date stamp
+    assert ref["move_history_after_bo"] == w._ggf_of(None, plies).split("BO[")[1]      # everything after the date stamp
 
 
-def test_resign_tuner_and_schedule_match_reference_worker(tmp_path):
+def test_resign_tuner_and_schedule_match_reference_worker(tmp_path, ref_host):
     """The UNMODIFIED reference SelfPlayWorker.finish_game / check_and_update_resignation_threshold /
-    decide_simulation_num_per_move (worker/self_play.py:219-272), called as plain functions on a stand-in `self`, against
-    the mirror over random game sequences.  Runs where the reference checkout exists."""
-    import oracle.ref_shims.install as shims
-    if not shims.available():
-        pytest.skip("reference sources not present")
-    shims.install()
-    from reversi_zero.worker.self_play import SelfPlayWorker as Ref
-    from reversi_zero.env.reversi_env import Winner
+    decide_simulation_num_per_move (worker/self_play.py:219-272), called as plain functions on a stand-in `self` over a
+    seeded sequence of 1500 games, against the mirror fed the same sequence: threshold and counters after every game."""
+    ref = ref_host["worker"]
     cfg, w = make_worker(tmp_path)
-    cfg.play.resign_threshold, cfg.play.false_positive_threshold, cfg.play.resign_threshold_delta = -0.8, 0.05, 0.01
-
-    class RefSelf:     # what the reference methods touch
-        pass
-    r = RefSelf()
-    r.config = types.SimpleNamespace(play=types.SimpleNamespace(resign_threshold=-0.8, false_positive_threshold=0.05, resign_threshold_delta=0.01,
-                                                                 schedule_of_simulation_num_per_move=[(0, 8), (300, 50), (2000, 200)]),
-                                     resource=types.SimpleNamespace(force_simulation_num_file=str(tmp_path / "ref_force_sim")))
-    r.resign_test_game_count = r.false_positive_count_of_resign = 0
-    r.check_and_update_resignation_threshold = lambda: Ref.check_and_update_resignation_threshold(r)
-    r.reset_false_positive_count = lambda: Ref.reset_false_positive_count(r)
-    type(r).false_positive_rate = Ref.false_positive_rate
-    rng = np.random.default_rng(9)
-    winners = {1: Winner.black, 2: Winner.white, 3: Winner.draw}
-    for i in range(1500):
-        winner = int(rng.integers(1, 4))
-        mask = int(rng.integers(0, 4)) if rng.random() < 0.2 else 0
-        enabled = bool(rng.random() < 0.4)
-        player = lambda bit: types.SimpleNamespace(resigned=bool(mask & bit), finish_game=lambda z: None)   # noqa: E731
-        r.env = types.SimpleNamespace(winner=winners[winner])
-        r.black, r.white = player(1), player(2)
-        Ref.finish_game(r, resign_enabled=enabled)
-        w._finish_game(game(winner=winner, resigned_mask=mask, resign_enabled=int(enabled)))
-        assert abs(cfg.play.resign_threshold - r.config.play.resign_threshold) < 1e-12, i
-        assert (w.resign_test_game_count, w.false_positive_count_of_resign) == (r.resign_test_game_count, r.false_positive_count_of_resign), i
+    st = ref["start"]
+    cfg.play.resign_threshold, cfg.play.false_positive_threshold, cfg.play.resign_threshold_delta = (
+        st["resign_threshold"], st["false_positive_threshold"], st["resign_threshold_delta"])
+    assert len(ref["games"]) == len(ref["after"]) == 1500
+    for i, ((winner, mask, enabled), (threshold, n_test, n_fp)) in enumerate(zip(ref["games"], ref["after"])):
+        w._finish_game(game(winner=winner, resigned_mask=mask, resign_enabled=enabled))
+        assert abs(cfg.play.resign_threshold - threshold) < 1e-12, i
+        assert (w.resign_test_game_count, w.false_positive_count_of_resign) == (n_test, n_fp), i
     assert abs(cfg.play.resign_threshold - (-0.8)) > 0.005          # the threshold did move during the sequence
     # schedule + .force-sim override
-    cfg.play.schedule_of_simulation_num_per_move = [[0, 8], [300, 50], [2000, 200]]
-    for idx in (0, 1, 299, 300, 301, 1999, 2000, 123456):
-        assert w.decide_simulation_num_per_move(idx) == Ref.decide_simulation_num_per_move(r, idx)
-    for text in ("77\n", "0", "abc", ""):
-        for path in (cfg.resource.force_simulation_num_file, r.config.resource.force_simulation_num_file):
-            with open(path, "wt") as f:
-                f.write(text)
-        for idx in (0, 5000):
-            assert w.decide_simulation_num_per_move(idx) == Ref.decide_simulation_num_per_move(r, idx), (text, idx)
+    cfg.play.schedule_of_simulation_num_per_move = ref["schedule"]
+    for idx, sims in zip(ref["schedule_index"], ref["schedule_sims"], strict=True):
+        assert w.decide_simulation_num_per_move(idx) == sims
+    assert [text for text, _ in ref["force_file"]] == ["77\n", "0", "abc", ""]
+    for text, cases in ref["force_file"]:
+        with open(cfg.resource.force_simulation_num_file, "wt") as f:
+            f.write(text)
+        for idx, sims in cases:
+            assert w.decide_simulation_num_per_move(idx) == sims, (text, idx)
 
 
-def test_config_mirror_matches_reference_defaults_and_yaml():
+def reference_yml_configs(ref_host, tmp_path):
+    """-> [(what the reference's Config held after overlaying one of its config/*.yml files, the mirror's Config loaded
+    from the same YAML mapping)]"""
+    import yaml
+    from reversi_zero_b200.config import load_yaml
+    out = []
+    for name, ref in sorted(ref_host["config"]["yml"].items()):
+        path = tmp_path / name
+        path.write_text(yaml.safe_dump(ref["mapping"]))
+        out.append((ref, load_yaml(str(path), project_dir="/tmp/rz_proj")))
+    assert [name for name in sorted(ref_host["config"]["yml"])] == ["alpha_go_zero.yml", "alt.yml", "ch5.yml", "mini.yml"]
+    return out
+
+
+def test_config_mirror_matches_reference_defaults_and_yaml(tmp_path, ref_host):
     """Every attribute of the reference's Config() sections this path reads (config.py: resource paths relative to the
     project dir, model, play, play_data) has the same default in the mirror, and the reference's own config/*.yml files
-    overlay to the same values through both loaders.  Runs where the reference checkout exists."""
-    import oracle.ref_shims.install as shims
-    if not shims.available():
-        pytest.skip("reference sources not present")
-    shims.install()
-    import yaml
-    from moke_config import create_config as ref_create
-    from reversi_zero.config import Config as RefConfig
-    from reversi_zero_b200.config import load_yaml
-
+    overlay to the same values through both loaders."""
     def plain(v):
         return [plain(x) for x in v] if isinstance(v, (list, tuple)) else v
 
     def compare(ref, mine, sections):
         for sec in sections:
-            rs, ms = getattr(ref, sec), getattr(mine, sec)
-            for k, v in vars(rs).items():
+            ms = getattr(mine, sec)
+            assert ref[sec], sec
+            for k, v in ref[sec].items():
                 if sec == "resource":
-                    if isinstance(v, str) and os.sep in v:        # absolute paths: compare relative to the project dir
-                        assert os.path.relpath(getattr(ms, k), mine.resource.project_dir) == os.path.relpath(v, ref.resource.project_dir), k
-                    elif not isinstance(v, str):
-                        continue
+                    if isinstance(v, dict):        # absolute paths: compare relative to the project dir
+                        assert os.path.relpath(getattr(ms, k), mine.resource.project_dir) == v["relpath"], k
                     else:
                         assert getattr(ms, k) == v, k
                 else:
-                    assert plain(getattr(ms, k)) == plain(v), (sec, k)
+                    assert plain(getattr(ms, k)) == v, (sec, k)
 
-    compare(RefConfig(), Config(project_dir="/tmp/rz_proj"), ("resource", "model", "play", "play_data"))
-    cfg_dir = "/root/reference/config"
-    for name in sorted(os.listdir(cfg_dir)):
-        if not name.endswith(".yml"):
-            continue
-        with open(os.path.join(cfg_dir, name), "rt") as f:
-            ref = ref_create(RefConfig, yaml.safe_load(f))
-        mine = load_yaml(os.path.join(cfg_dir, name), project_dir="/tmp/rz_proj")
+    compare(ref_host["config"]["defaults"], Config(project_dir="/tmp/rz_proj"), ("resource", "model", "play", "play_data"))
+    for ref, mine in reference_yml_configs(ref_host, tmp_path):
         compare(ref, mine, ("model", "play", "play_data"))
 
 
-def test_eval_play_config_matches_reference_effective_settings():
+def test_eval_play_config_matches_reference_effective_settings(tmp_path, ref_host):
     """What an evaluation game runs with: the reference's EvaluateConfig.play_config (a fresh PlayConfig + five overrides +
     the YAML's eval.play_config), except the three fields ReversiPlayer reads from config.play even then
     (agent/player.py:127,237-238,264) -- for the defaults and every config/*.yml of the reference."""
-    import oracle.ref_shims.install as shims
-    if not shims.available():
-        pytest.skip("reference sources not present")
-    shims.install()
-    import yaml
-    from moke_config import create_config as ref_create
-    from reversi_zero.config import Config as RefConfig
-    from reversi_zero_b200.config import load_yaml
-    cases = [(RefConfig(), Config(project_dir="/tmp/rz_proj"))]
-    for name in sorted(os.listdir("/root/reference/config")):
-        if name.endswith(".yml"):
-            with open(os.path.join("/root/reference/config", name), "rt") as f:
-                cases.append((ref_create(RefConfig, yaml.safe_load(f)), load_yaml(os.path.join("/root/reference/config", name), project_dir="/tmp/rz_proj")))
+    cases = [(ref_host["config"]["defaults"], Config(project_dir="/tmp/rz_proj"))] + reference_yml_configs(ref_host, tmp_path)
     for ref, mine in cases:
-        want = dict(vars(ref.eval.play_config))
-        for k in ("allowed_resign_turn", "use_solver_turn_in_simulation", "virtual_loss"):
-            want[k] = getattr(ref.play, k)
+        want = dict(ref["eval_play_config"])
+        want.update(ref["play_fields"])
+        assert sorted(ref["play_fields"]) == ["allowed_resign_turn", "use_solver_turn_in_simulation", "virtual_loss"]
         got = vars(eval_play_config(mine))
         for k, v in want.items():
             if k == "share_mtcs_info_in_self_play":
@@ -334,8 +293,10 @@ def test_eval_play_config_matches_reference_effective_settings():
             gv = got[k]
             norm = (lambda x: [list(y) for y in x]) if k == "schedule_of_simulation_num_per_move" else (lambda x: x)
             assert norm(gv) == norm(v), (getattr(ref, "type", "?"), k)
-        # the reference's own Config object is accepted as well
-        got2 = vars(eval_play_config(ref))
+        # the reference's own Config object is accepted as well: its eval.play_config and play sections as attributes
+        ref_obj = types.SimpleNamespace(eval=types.SimpleNamespace(play_config=types.SimpleNamespace(**ref["eval_play_config"])),
+                                        play=types.SimpleNamespace(**ref["play_fields"]))
+        got2 = vars(eval_play_config(ref_obj))
         assert all(got2[k] == want[k] for k in want if k not in ("share_mtcs_info_in_self_play",))
 
 

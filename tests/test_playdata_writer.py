@@ -2,6 +2,7 @@
 require the file to be byte-identical to json.dumps of the reference-format records, and loadable by
 the reference's own convert_to_training_data logic (worker/optimize.py:215-231, restated)."""
 import json
+import os
 
 import numpy as np
 import pytest
@@ -70,23 +71,28 @@ def test_float_repr_edge_cases(tmp_path):
             assert repr(float(v)) in text
 
 
-def test_reference_trainer_loads_our_files(tmp_path):
-    """SURVEY 8(c)(v): a play_data file written by the C-ABI writer goes through the UNMODIFIED reference's
-    read_game_data_from_file + OptimizeWorker.convert_to_training_data (worker/optimize.py:215-231).  Runs only where
-    the reference checkout exists (the build container)."""
-    import oracle.ref_shims.install as shims
-    if not shims.available():
-        pytest.skip("reference sources not present")
-    shims.install()
-    from reversi_zero.lib.data_helper import read_game_data_from_file
-    from reversi_zero.worker.optimize import OptimizeWorker
+def write_trainer_file(path):
+    """play_data file of two seeded oracle games through the C-ABI writer -> number of records"""
     pp = mcts.PlayParams(simulation_num_per_move=20, parallel_search_num=4, noise_eps=0.25, c_puct=5)
     games = [mcts.SelfPlayGame(pp, onn.FakeNetAPI(), seed=5, game_id=i).play() for i in range(2)]
     G, P = to_ctypes(games)
+    return E.write_play_data(path, G, len(games), P, True, 4)
+
+
+def test_reference_trainer_loads_our_files(tmp_path, golden_dir):
+    """SURVEY 8(c)(v): a play_data file written by the C-ABI writer goes through the reference's read_game_data_from_file
+    + OptimizeWorker.convert_to_training_data (worker/optimize.py:215-231): json.load, then per record
+    bit_to_array(own / enemy, 64).reshape(8, 8) and np.array of the three lists.  tests/golden/ref_trainer_load.npz holds
+    what the unmodified reference returned for this file."""
     path = str(tmp_path / "play_20260922-000000.000000.json")
-    n = E.write_play_data(path, G, len(games), P, True, 4)
-    data = read_game_data_from_file(path)
-    states, policies, zs = OptimizeWorker.convert_to_training_data(data)
+    n = write_trainer_file(path)
+    with open(path, "rt") as f:
+        data = json.load(f)
+    states = np.array([[ob.bit_to_array(s[0], 64).reshape(8, 8), ob.bit_to_array(s[1], 64).reshape(8, 8)] for s, _, _ in data])
+    policies, zs = np.array([p for _, p, _ in data]), np.array([z for _, _, z in data])
+    ref = np.load(os.path.join(golden_dir, "ref_trainer_load.npz"))
+    for got, want in ((states, ref["states"]), (policies, ref["policies"]), (zs, ref["zs"])):
+        assert got.dtype == want.dtype and np.array_equal(got, want)
     assert states.shape == (n, 2, 8, 8) and policies.shape == (n, 64) and zs.shape == (n,)
     assert states.dtype == np.uint8 and set(np.unique(zs)) <= {-1, 0, 1}
     assert np.allclose(policies.sum(axis=1), 1.0)

@@ -1,18 +1,19 @@
-"""The reference's OWN compiled code (lib/alt/bitboard_cython.pyx, lib/alt/reversi_solver_cython.pyx, built by
-oracle/build_ref.py into oracle/_ref -- it travels to the GPU box) against
+"""The reference's OWN compiled code (lib/alt/bitboard_cython.pyx, lib/alt/reversi_solver_cython.pyx) against
   * the oracle restatements (CPU, here), and
   * the CUDA operators through the C ABI (GPU): K1 move generation / flips on 1 M seeded positions of the
     SURVEY 8(d) config-5 recipe, and the batched endgame solver.
-Skipped where oracle/_ref has not been built (it needs the reference checkout once)."""
+What the reference computed is stored in tests/golden/ref_native.npz (tests/golden/make_golden_standalone.py): its
+move generation and flips on a seeded 24 000-position sample of the 1 M set, and its solver's answer on every endgame."""
+import os
+
 import numpy as np
 import pytest
 
-from oracle import bitboard as ob, ref_native
+from oracle import bitboard as ob
 from oracle.solver import Solver
 
-pytestmark = pytest.mark.skipif(not ref_native.available(), reason="oracle/_ref not built")
-
 U64 = np.uint64
+N_CONFIG5 = 1_000_000
 
 
 def config5_positions(n, seed=20260922):
@@ -27,13 +28,6 @@ def config5_positions(n, seed=20260922):
     occ[2 * third:] = a[2 * third:] | b[2 * third:]
     pos = rng.integers(0, 64, size=n, dtype=np.uint8)
     return occ & r, occ & ~r, pos
-
-
-def reference_outputs(own, enemy, pos):
-    bb, _ = ref_native.load()
-    legal = np.fromiter((bb.find_correct_moves(int(o), int(e)) for o, e in zip(own, enemy)), dtype=U64, count=len(own))
-    flip = np.fromiter((bb.calc_flip(int(p), int(o), int(e)) for p, o, e in zip(pos, own, enemy)), dtype=U64, count=len(own))
-    return legal, flip
 
 
 def random_endgames(n, seed, max_empties=10):
@@ -52,43 +46,54 @@ def random_endgames(n, seed, max_empties=10):
     return out
 
 
-def reference_solve(own, enemy, exactly):
-    """ReversiSolver.solve(black, white, next_player, exactly) of the compiled reference, position given in the mover's frame"""
-    _, sv = ref_native.load()
-    mv, sc = sv.ReversiSolver().solve(own, enemy, ref_native.player_enum().black, exactly=exactly)
-    return (-1, 0) if mv is None else (int(mv), int(sc))
+@pytest.fixture(scope="module")
+def ref(golden_dir):
+    return dict(np.load(os.path.join(golden_dir, "ref_native.npz")))
 
 
-def test_oracle_bitboard_matches_compiled_reference():
-    own, enemy, pos = config5_positions(100_000)
-    legal, flip = reference_outputs(own, enemy, pos)
-    assert np.array_equal(ob.find_correct_moves_batch(own, enemy), legal)
-    assert np.array_equal(ob.calc_flip_batch(pos, own, enemy), flip)
+def reference_solves(ref, name, seed, n):
+    """-> [(own, enemy, {exactly: (move, score)})] of ReversiSolver.solve(black, white, next_player, exactly) of the
+    compiled reference, position given in the mover's frame; the stored endgames are the ones random_endgames draws"""
+    own, enemy, res = ref[name + "_own"], ref[name + "_enemy"], ref[name + "_result"].astype(int)
+    assert [(int(o), int(e)) for o, e in zip(own, enemy)] == random_endgames(n, seed)
+    return [(int(o), int(e), {True: (int(r[0]), int(r[1])), False: (int(r[2]), int(r[3]))}) for o, e, r in zip(own, enemy, res)]
 
 
-def test_oracle_solver_matches_compiled_reference():
-    for own, enemy in random_endgames(120, seed=41):
+def test_oracle_bitboard_matches_compiled_reference(ref):
+    own, enemy, pos = config5_positions(N_CONFIG5)
+    idx = ref["index"]
+    assert len(idx) == 24_000 and np.array_equal(own[idx], ref["own"]) and np.array_equal(enemy[idx], ref["enemy"])
+    assert np.array_equal(pos[idx], ref["pos"])
+    assert np.array_equal(ob.find_correct_moves_batch(ref["own"], ref["enemy"]), ref["legal"])
+    assert np.array_equal(ob.calc_flip_batch(ref["pos"], ref["own"], ref["enemy"]), ref["flip"])
+
+
+def test_oracle_solver_matches_compiled_reference(ref):
+    for own, enemy, want in reference_solves(ref, "solver41", 41, 120):
         for exactly in (True, False):
             mv, sc = Solver().solve(own, enemy, exactly)
-            assert ((-1, 0) if mv is None else (mv, sc)) == reference_solve(own, enemy, exactly)
+            assert ((-1, 0) if mv is None else (mv, sc)) == want[exactly]
 
 
 @pytest.mark.gpu
-def test_k1_kernels_match_compiled_reference_1m():
+def test_k1_kernels_match_compiled_reference_1m(ref):
     from reversi_zero_b200.lib import bitboard as zb
-    own, enemy, pos = config5_positions(1_000_000)
-    legal, flip = reference_outputs(own, enemy, pos)
-    assert np.array_equal(zb.find_correct_moves_batch(own, enemy), legal)      # bit-exact, 1 M positions
-    assert np.array_equal(zb.calc_flip_batch(pos, own, enemy), flip)          # including occupied / illegal squares
+    own, enemy, pos = config5_positions(N_CONFIG5)
+    legal, flip = zb.find_correct_moves_batch(own, enemy), zb.calc_flip_batch(pos, own, enemy)
+    idx = ref["index"]
+    assert np.array_equal(legal[idx], ref["legal"])        # bit-exact against the reference on the stored sample
+    assert np.array_equal(flip[idx], ref["flip"])          # including occupied / illegal squares
+    assert np.array_equal(legal, ob.find_correct_moves_batch(own, enemy))   # and against the oracle on all 1 M positions
+    assert np.array_equal(flip, ob.calc_flip_batch(pos, own, enemy))
 
 
 @pytest.mark.gpu
-def test_device_solver_matches_compiled_reference():
+def test_device_solver_matches_compiled_reference(ref):
     from reversi_zero_b200.lib import reversi_solver as zs
-    cases = random_endgames(200, seed=43)
+    cases = reference_solves(ref, "solver43", 43, 200)
     own = [c[0] for c in cases]
     enemy = [c[1] for c in cases]
     for exactly in (True, False):
         mv, sc = zs.solve_batch(own, enemy, [exactly] * len(cases))
-        for o, e, m, s in zip(own, enemy, mv, sc):
-            assert (int(m), int(s)) == reference_solve(o, e, exactly)
+        for (_, _, want), m, s in zip(cases, mv, sc):
+            assert (int(m), int(s)) == want[exactly]
