@@ -37,7 +37,7 @@ extern "C" {
 #define RZ_ECAPACITY (-5) /* an engine arena overflowed (nodes / edges / records) */
 #define RZ_EIO (-6)      /* file I/O failed */
 
-#define RZ_ABI_VERSION 2
+#define RZ_ABI_VERSION 3
 
 int rz_abi_version(void);
 const char* rz_last_error(void);
@@ -114,11 +114,6 @@ typedef struct rz_net_cfg {
 #define RZ_NET_IMPL_GENERIC 1 /* CUDA-core fp32 kernel, any configuration */
 #define RZ_NET_IMPL_TCGEN05 2 /* fused persistent tcgen05 tower (filters must be 256) */
 
-/* Which kernel serves RZ_NET_IMPL_TCGEN05 from now on (process-wide): 1 = one CTA per tile (csrc/rz_net_tc.cu),
- * 2 = CTA pairs, cta_group::2, epilogue overlapped with the MMA stream (csrc/rz_net_tc2.cu).  The default comes from
- * the environment variable RZ_TOWER_KERNEL when the first network call is made (default 2).  Used by the tests and benchmarks to
- * run both on the same inputs. */
-int rz_net_set_tower_kernel(int version);
 int rz_net_create(const rz_net_cfg* cfg, int device, rz_net** out);
 int rz_net_destroy(rz_net* net);
 /* number of float32 values in the weight blob for this configuration.  Blob layout (Keras tensor

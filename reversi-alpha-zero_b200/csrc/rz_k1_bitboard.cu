@@ -14,7 +14,7 @@
 #include <string.h>
 #include "rz_bitboard.cuh"
 #include "rz_bitsliced.cuh"
-#include "rz_tc_common.cuh"   // mbarrier / bulk-copy wrappers
+#include "rz_ptx.cuh"   // mbarrier / bulk-copy wrappers
 #include "rz_common.cuh"
 
 namespace rz {
@@ -89,8 +89,8 @@ template <bool FLIP>
 __global__ void __launch_bounds__(kThreads, 1) k1_bs_staged(const uint8_t* __restrict__ pos, const u64* __restrict__ own,
                                                             const u64* __restrict__ enemy, u64* __restrict__ out, size_t n_tiles) {
     extern __shared__ uint8_t k1_smem_raw[];
-    const uint32_t base = (tc::smem_u32(k1_smem_raw) + 127u) & ~127u;
-    uint8_t* sm = k1_smem_raw + (base - tc::smem_u32(k1_smem_raw));
+    const uint32_t base = (ptx::smem_u32(k1_smem_raw) + 127u) & ~127u;
+    uint8_t* sm = k1_smem_raw + (base - ptx::smem_u32(k1_smem_raw));
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const size_t warp = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((size_t)gridDim.x * blockDim.x) >> 5;
     const uint32_t bar = base + (kThreads / 32) * kStagePerWarp + w * 8;
@@ -99,22 +99,22 @@ __global__ void __launch_bounds__(kThreads, 1) k1_bs_staged(const uint8_t* __res
     const u64* se = so + 1024;
     const uint8_t* sp = sm + w * kStagePerWarp + 16384;
     if (lane == 0) {
-        tc::mbar_init(bar, 1);
+        ptx::mbar_init(bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncwarp();
     auto fetch = [&](size_t t) {   // lane 0 only
-        tc::mbar_expect_tx(bar, FLIP ? 16384u + 1024u : 16384u);
-        tc::bulk_g2s(s_own, own + t * 1024, 8192, bar);
-        tc::bulk_g2s(s_en, enemy + t * 1024, 8192, bar);
-        if (FLIP) tc::bulk_g2s(s_pos, pos + t * 1024, 1024, bar);
+        ptx::mbar_expect_tx(bar, FLIP ? 16384u + 1024u : 16384u);
+        ptx::bulk_g2s(s_own, own + t * 1024, 8192, bar);
+        ptx::bulk_g2s(s_en, enemy + t * 1024, 8192, bar);
+        if (FLIP) ptx::bulk_g2s(s_pos, pos + t * 1024, 1024, bar);
     };
     uint32_t phase = 0;
     if (warp < n_tiles && lane == 0) fetch(warp);
     for (size_t t = warp; t < n_tiles; t += n_warps) {
         u64 o[32], e[32], r[32];
         uint8_t ps[32];
-        tc::mbar_wait(bar, phase);
+        ptx::mbar_wait(bar, phase);
         phase ^= 1;
 #pragma unroll
         for (int i = 0; i < 32; ++i) {
@@ -129,7 +129,7 @@ __global__ void __launch_bounds__(kThreads, 1) k1_bs_staged(const uint8_t* __res
             for (int i = 0; i < 32; ++i) out[ob + i * 32] = calc_flip(sp[i * 32 + lane] & 63, so[i * 32 + lane], se[i * 32 + lane]);
         __syncwarp();                       // every lane is done with the staging buffer: it may be refilled
         if (lane == 0 && t + n_warps < n_tiles) {
-            tc::fence_proxy_async();
+            ptx::fence_proxy_async();
             fetch(t + n_warps);
         }
         if (scalar_path) continue;

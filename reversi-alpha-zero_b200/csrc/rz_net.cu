@@ -183,8 +183,7 @@ int net_forward(rz_net* net, const uint64_t* own, const uint64_t* enemy, float* 
     if (impl == RZ_NET_IMPL_AUTO) impl = net->cfg.filters == 256 ? RZ_NET_IMPL_TCGEN05 : RZ_NET_IMPL_GENERIC;
     if (impl == RZ_NET_IMPL_TCGEN05) {
         RZ_REQUIRE(net->cfg.filters == 256, "tcgen05 tower requires filters == 256 (got %d)", net->cfg.filters);
-        return tower_kernel_version() == 2 ? net_forward_tc2(net, own, enemy, policy, value, n, stream, nullptr)
-                                           : net_forward_tc(net, own, enemy, policy, value, n, stream, nullptr);
+        return net_forward_tc(net, own, enemy, policy, value, n, stream, nullptr);
     }
     RZ_REQUIRE(impl == RZ_NET_IMPL_GENERIC, "unknown net impl %d", impl);
     return net_forward_generic(net, own, enemy, policy, value, n, stream);
@@ -195,8 +194,7 @@ int net_forward_counted(rz_net* net, const uint64_t* own, const uint64_t* enemy,
     if (!net->loaded) { set_error("rz_net: weights not loaded"); return RZ_ESTATE; }
     if (impl == RZ_NET_IMPL_AUTO) impl = net->cfg.filters == 256 ? RZ_NET_IMPL_TCGEN05 : RZ_NET_IMPL_GENERIC;
     if (impl == RZ_NET_IMPL_TCGEN05)
-        return tower_kernel_version() == 2 ? net_forward_tc2(net, own, enemy, policy, value, max_n, stream, nullptr, count_dev)
-                                           : net_forward_tc(net, own, enemy, policy, value, max_n, stream, nullptr, count_dev);
+        return net_forward_tc(net, own, enemy, policy, value, max_n, stream, nullptr, count_dev);
     return net_forward_generic(net, own, enemy, policy, value, max_n, stream, count_dev);
 }
 
@@ -213,19 +211,10 @@ static int finish_load(rz_net* net, cudaStream_t stream) {
     fold_bn_kernel<<<1, 32, 0, stream>>>(net->blob, net->off_policy_conv, (size_t)F * 2, 2, ssh, ssh + 2);
     fold_bn_kernel<<<1, 32, 0, stream>>>(net->blob, net->off_value_conv, (size_t)F, 1, ssh + 4, ssh + 5);
     RZ_LAUNCH_CHECK();
-    if (F == 256) { RZ_TRY(net_pack_tc(net, stream)); RZ_TRY(net_pack_tc2(net, stream)); }
+    if (F == 256) RZ_TRY(net_pack_tc(net, stream));
     RZ_CUDA_TRY(cudaStreamSynchronize(stream));
     net->loaded = true;
     return RZ_OK;
-}
-
-static int g_tower_kernel = 0;
-int tower_kernel_version() {
-    if (g_tower_kernel == 0) {
-        const char* s = getenv("RZ_TOWER_KERNEL");
-        g_tower_kernel = (s && atoi(s) == 1) ? 1 : 2;   // default: the CTA-pair kernel (30.9 ms vs 35.2 ms per 32 768 positions)
-    }
-    return g_tower_kernel;
 }
 
 }  // namespace rz
@@ -262,10 +251,8 @@ int rz_net_create(const rz_net_cfg* cfg, int device, rz_net** out) {
     cudaError_t e = cudaMalloc(&net->blob, off * sizeof(float));
     if (e == cudaSuccess) e = cudaMalloc(&net->scale_shift, ss_floats(*cfg) * sizeof(float));
     if (e == cudaSuccess && F == 256) {
-        e = cudaMalloc(&net->tc_w0, (size_t)4 * 256 * 8 * sizeof(__half));
-        if (e == cudaSuccess && R > 0) e = cudaMalloc(&net->tc_w, (size_t)2 * R * 36 * 8 * 256 * 8 * sizeof(__half));
-        if (e == cudaSuccess) e = cudaMalloc(&net->tc2_w0, (size_t)2 * 2 * 4 * 64 * 8 * sizeof(__half));
-        if (e == cudaSuccess && R > 0) e = cudaMalloc(&net->tc2_w, (size_t)2 * R * 36 * 2 * 8192 * sizeof(__half));
+        e = cudaMalloc(&net->tc_w0, (size_t)2 * 2 * 4 * 64 * 8 * sizeof(__half));
+        if (e == cudaSuccess && R > 0) e = cudaMalloc(&net->tc_w, (size_t)2 * R * 36 * 2 * 8192 * sizeof(__half));
     }
     if (e != cudaSuccess) {
         set_error("rz_net_create: cudaMalloc failed: %s", cudaGetErrorString(e));
@@ -280,7 +267,7 @@ int rz_net_create(const rz_net_cfg* cfg, int device, rz_net** out) {
 int rz_net_destroy(rz_net* net) {
     if (!net) return RZ_OK;
     cudaSetDevice(net->device);
-    cudaFree(net->blob); cudaFree(net->scale_shift); cudaFree(net->tc_w0); cudaFree(net->tc_w); cudaFree(net->tc2_w0); cudaFree(net->tc2_w); cudaFree(net->scratch);
+    cudaFree(net->blob); cudaFree(net->scale_shift); cudaFree(net->tc_w0); cudaFree(net->tc_w); cudaFree(net->scratch);
     delete net;
     return RZ_OK;
 }
@@ -307,12 +294,6 @@ int rz_net_load_weights_dev(rz_net* net, const float* blob_dev, size_t n_floats,
     return finish_load(net, (cudaStream_t)stream);
 }
 
-int rz_net_set_tower_kernel(int version) {
-    RZ_REQUIRE(version == 1 || version == 2, "rz_net_set_tower_kernel: version must be 1 or 2");
-    g_tower_kernel = version;
-    return RZ_OK;
-}
-
 int rz_net_predict_dev(rz_net* net, const uint64_t* own, const uint64_t* enemy, float* policy, float* value, size_t n, int impl,
                        void* stream) {
     RZ_REQUIRE(net && (n == 0 || (own && enemy && policy && value)), "rz_net_predict_dev: null pointer");
@@ -323,17 +304,14 @@ int rz_net_debug_tower_dev(rz_net* net, const uint64_t* own, const uint64_t* ene
                            void* stream) {
     RZ_REQUIRE(net && own && enemy && policy && value && tower, "rz_net_debug_tower_dev: null pointer");
     if (!net->loaded) { set_error("rz_net: weights not loaded"); return RZ_ESTATE; }
-    return tower_kernel_version() == 2 ? net_forward_tc2(net, own, enemy, policy, value, n, (cudaStream_t)stream, tower)
-                                       : net_forward_tc(net, own, enemy, policy, value, n, (cudaStream_t)stream, tower);
+    return net_forward_tc(net, own, enemy, policy, value, n, (cudaStream_t)stream, tower);
 }
 
 int rz_net_debug_heads_dev(rz_net* net, const uint64_t* own, const uint64_t* enemy, float* policy, float* value, float* tower,
                            float* policy_logits, float* value_logit, size_t n, void* stream) {
     RZ_REQUIRE(net && own && enemy && policy && value && policy_logits && value_logit, "rz_net_debug_heads_dev: null pointer");
     if (!net->loaded) { set_error("rz_net: weights not loaded"); return RZ_ESTATE; }
-    return tower_kernel_version() == 2
-               ? net_forward_tc2(net, own, enemy, policy, value, n, (cudaStream_t)stream, tower, nullptr, policy_logits, value_logit)
-               : net_forward_tc(net, own, enemy, policy, value, n, (cudaStream_t)stream, tower, nullptr, policy_logits, value_logit);
+    return net_forward_tc(net, own, enemy, policy, value, n, (cudaStream_t)stream, tower, nullptr, policy_logits, value_logit);
 }
 
 int rz_net_predict(rz_net* net, const uint8_t* planes, float* policy, float* value, size_t n, int impl) {

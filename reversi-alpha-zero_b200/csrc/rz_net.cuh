@@ -21,12 +21,9 @@ struct rz_net {
     size_t off_conv0, off_res0, res_stride_conv;  // kernel offset of conv0; of res0.conv1; floats per (conv+bn) group
     size_t off_policy_conv, off_policy_fc_k, off_policy_fc_b;
     size_t off_value_conv, off_value_fc1_k, off_value_fc1_b, off_value_fc2_k, off_value_fc2_b;
-    // tcgen05 tower (F == 256 only)
-    __half* tc_w0;       // [4 kc][256 n][8] fp16: layer-0 weights, K = 18 padded to 32, UMMA K-major no-swizzle image
-    __half* tc_w;        // [2R layers][36 stages][8 kc][256 n][8] fp16: one 32 KB shared-memory image per pipeline stage
-    // pair kernel (rz_net_tc2.cu, cta_group::2): the same weights in the order its K / N loops consume them
-    __half* tc2_w0;      // [cta 2][nh 2][kc 4][n 64][8]
-    __half* tc2_w;       // [2R layers][36 stages][cta 2][kbl 2][kc 8][n 64][8]: one 16 KB image per CTA and pipeline stage
+    // tcgen05 tower (F == 256 only, rz_net_tc.cu): fp16 UMMA K-major no-swizzle images in the order its K / N loops consume them
+    __half* tc_w0;       // [cta 2][nh 2][kc 4][n 64][8]: layer-0 weights, K = 18 padded to 32
+    __half* tc_w;        // [2R layers][36 stages][cta 2][kbl 2][kc 8][n 64][8]: one 16 KB image per CTA and pipeline stage
     // scratch for the host-buffer predict path
     void* scratch;
     size_t scratch_bytes;
@@ -43,19 +40,12 @@ int net_forward_generic(rz_net* net, const uint64_t* own, const uint64_t* enemy,
 // batch size known only on the device (count_dev), at most max_n
 int net_forward_counted(rz_net* net, const uint64_t* own, const uint64_t* enemy, float* policy, float* value,
                         const uint32_t* count_dev, size_t max_n, int impl, cudaStream_t stream);
+// the fused tcgen05 tower on CTA pairs (rz_net_tc.cu)
 int net_forward_tc(rz_net* net, const uint64_t* own, const uint64_t* enemy, float* policy, float* value, size_t n,
                    cudaStream_t stream, float* dbg_tower /* nullable: [n][64][256] fp32 tower output */,
                    const uint32_t* n_dev = nullptr /* nullable: actual batch size in device memory (<= n) */,
                    float* dbg_logits = nullptr /* nullable: [n][64] policy logits */, float* dbg_vlogit = nullptr /* nullable: [n] */);
 int net_pack_tc(rz_net* net, cudaStream_t stream);
-// the CTA-pair kernel (rz_net_tc2.cu); same contract as net_forward_tc
-int net_forward_tc2(rz_net* net, const uint64_t* own, const uint64_t* enemy, float* policy, float* value, size_t n,
-                    cudaStream_t stream, float* dbg_tower, const uint32_t* n_dev = nullptr, float* dbg_logits = nullptr,
-                    float* dbg_vlogit = nullptr);
-int net_pack_tc2(rz_net* net, cudaStream_t stream);
-// which tcgen05 tower kernel serves RZ_NET_IMPL_TCGEN05: 2 = CTA pairs with overlapped epilogue (default), 1 = one CTA per
-// tile (RZ_TOWER_KERNEL=1, rz_net_set_tower_kernel)
-int tower_kernel_version();
 int net_forward(rz_net* net, const uint64_t* own, const uint64_t* enemy, float* policy, float* value, size_t n, int impl,
                 cudaStream_t stream);
 

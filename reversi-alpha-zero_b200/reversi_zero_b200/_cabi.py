@@ -87,7 +87,6 @@ SIGNATURES = {
     "rz_net_load_weights": (C.c_int, [vp, f32p, sz]),
     "rz_net_load_weights_dev": (C.c_int, [vp, vp, sz, vp]),
     "rz_net_predict_dev": (C.c_int, [vp, vp, vp, vp, vp, sz, C.c_int, vp]),
-    "rz_net_set_tower_kernel": (C.c_int, [C.c_int]),
     "rz_net_debug_tower_dev": (C.c_int, [vp, vp, vp, vp, vp, vp, sz, vp]),
     "rz_net_debug_heads_dev": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]),
     "rz_net_predict": (C.c_int, [vp, u8p, f32p, f32p, sz, C.c_int]),

@@ -9,11 +9,6 @@ from .agent import model as M
 IMPL_AUTO, IMPL_GENERIC, IMPL_TCGEN05 = 0, 1, 2
 
 
-def set_tower_kernel(version):
-    """1 = one CTA per tile, 2 = CTA pairs with overlapped epilogue (rz_net_set_tower_kernel); process-wide"""
-    _cabi.check(_cabi.lib().rz_net_set_tower_kernel(int(version)), "rz_net_set_tower_kernel")
-
-
 class Net:
     def __init__(self, model_config, device=0):
         self.mc = model_config

@@ -14,7 +14,9 @@ from reversi_zero_b200.env.reversi_env import ReversiEnv, Player, Winner
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_of_abi_3():
+    """The library exports every symbol include/rz_engine.h declares, _cabi binds exactly those, and it reports ABI 3 (the
+    version without rz_net_set_tower_kernel)."""
     hdr = open(os.path.join(ROOT, "include", "rz_engine.h")).read()
     hdr = re.sub(r"/\*.*?\*/", "", hdr, flags=re.S)
     declared = set(re.findall(r"\b(rz_[a-z0-9_]+)\s*\(", hdr))
@@ -23,7 +25,7 @@ def test_library_exports_every_declared_symbol():
     missing = [n for n in sorted(declared) if not hasattr(lib, n)]
     assert not missing, f"symbols declared but not exported: {missing}"
     assert declared == set(_cabi.SIGNATURES), declared ^ set(_cabi.SIGNATURES)
-    assert lib.rz_abi_version() == 2
+    assert lib.rz_abi_version() == 3
 
 
 def test_host_twins_vs_golden(golden_dir):

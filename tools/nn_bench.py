@@ -45,10 +45,9 @@ def run(n=32768, iters=5, warmup=2, res_blocks=10):
 
 
 if __name__ == "__main__":
-    # python tools/nn_bench.py [res_blocks] [iters]; RZ_TOWER_EXPERIMENT=1|2 times the measurement variants of the kernel
+    # python tools/nn_bench.py [res_blocks] [iters]
     rb = int(sys.argv[1]) if len(sys.argv) > 1 else 10
     iters = int(sys.argv[2]) if len(sys.argv) > 2 else 5
     for n in (296, 32768):
         r = run(n, iters=iters, res_blocks=rb)
-        r["experiment"] = os.environ.get("RZ_TOWER_EXPERIMENT", "0")
         print(json.dumps(r))

@@ -8,7 +8,7 @@ tower is computed EXACTLY (fp64) on operands rounded the way a format would roun
 residual stream, heads) in fp32 -- so a row is the floor of what any kernel using that format can reach (tools/nn_diag.py
 shows that the tcgen05 kernel sits on its format's floor).
 
-    fp16            both operands rounded to fp16 (what csrc/rz_net_tc2.cu does: 1 MMA per product)
+    fp16            both operands rounded to fp16 (what csrc/rz_net_tc.cu does: 1 MMA per product)
     fp16-scaled     activations multiplied by a per-layer power of two that brings their maximum to 2^14 before rounding
                     (proposal 1; fp16 rounding is relative, so nothing changes unless values were subnormal)
     bf16            both operands rounded to bf16
